@@ -25,6 +25,7 @@ import time
 
 ROOT = pathlib.Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (which may be read-only)
 
 METRIC = "streaming frames/sec (10 tok/frame, 12k-ctx KV), all GPUs"
 UNIT = "frames/s"
@@ -65,6 +66,22 @@ def _peaks():
         d = json.loads(p.read_text())
         return float(d["hbm_gbs"]), float(d.get("bf16_tflops_sustained", d.get("bf16_tflops", 1468.8))), "measured"
     return 6650.0, 1400.0, "fallback"
+
+
+def dump_outputs(out_dir, frame_embeds, logits, decisions):
+    """--dump-outputs: what the last timed frame step handed its caller, as .npy files: frame_embeds.npy (float32
+    [10, hidden], the ViT + connector output the step consumed), logits.npy (float32 [1, vocab], last position) and one
+    float64 decision_<field>.npy per field of the on-device speak/silent decision."""
+    import numpy as np
+    import torch
+    from videollm_online_b200.engine import Decision
+    row = decisions[0].cpu()
+    dec = Decision(row, row.view(torch.float32))
+    arrays = {"frame_embeds": frame_embeds.float().cpu().numpy(), "logits": logits.float().cpu().numpy()}
+    arrays.update({"decision_" + f: np.array([getattr(dec, f)], dtype=np.float64) for f in Decision.__slots__})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -336,10 +353,11 @@ def run_engine_arm(args):
     pre_evs = [torch.cuda.Event(), torch.cuda.Event()]
 
     def pipelined(n, base, from_host=False, read_back=False, step_fn=None):
-        """n frame steps; the ViT runs D frames at a time on the side stream, one group ahead of the decoder"""
+        """n frame steps; the ViT runs D frames at a time on the side stream, one group ahead of the decoder.
+        Returns what the last step's eng.step returned (without step_fn): its logits and decisions on the device."""
         n_groups = (n + D - 1) // D
         encode_on_side(base, 0, from_host, count=min(D, n))
-        fe = None
+        fe = res = None
         for i in range(n):
             g, j = divmod(i, D)
             if j == 0:
@@ -354,11 +372,12 @@ def run_engine_arm(args):
                 step_fn(i, fe[10 * j:10 * j + 10])
             else:
                 packed[1:] = fe[10 * j:10 * j + 10]
-                eng.step([sid], [11], packed, row_ids=prefix, want_logits=True)
+                res = eng.step([sid], [11], packed, row_ids=prefix, want_logits=True)
             if j == 0 and g + 1 < n_groups:
                 encode_on_side(base + (g + 1) * D, (g + 1) & 1, from_host, after=pre_evs[g & 1], count=min(D, n - (g + 1) * D))
             if read_back:
                 eng.read_decisions(1)
+        return res
 
     # ---- device-resident timing (value)
     eng.kv_fill_synthetic(sid, KV_START, seed=7 + rank)
@@ -371,9 +390,11 @@ def run_engine_arm(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record(stream)
-    pipelined(K, Wm)
+    last_logits, last_dec = pipelined(K, Wm)
     e1.record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, packed[1:], last_logits, last_dec)
     ms_total = reduce_max(e0.elapsed_time(e1))
     launches = eng.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
@@ -768,7 +789,14 @@ def main():
                          "co-resides with the decoder step; >= 3 = 2-CTA tensor-bound GEMMs, serialised against the step)")
     ap.add_argument("--no-extras", dest="extras", action="store_false", help="skip the side measurements of the other BASELINE configs")
     ap.add_argument("--quick-extras", dest="quick_extras", action="store_true", help="shorter side measurements (dev runs)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write what the last timed frame step computed (frame embeddings, logits, decision) to DIR/<name>.npy; "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA engine's outputs; the reference arm has none")
     with _StdoutToStderr() as guard:
         line = run_reference_arm(args) if args.impl == "reference" else run_engine_arm(args)
     if line is not None:

@@ -1,15 +1,20 @@
 """Generate the golden fixtures by RUNNING THE REFERENCE's own modules (CPU) on seeded inputs.
 
-    python tests/golden/make_golden.py            # needs /root/reference + transformers; build container only
+    python tests/golden/make_golden.py            # tiny_reference.pt
+    python tests/golden/make_golden.py forward    # reference_forward.json: digests of the reference's forward on this host
+    python tests/golden/make_golden.py clips      # demo_{bicycle,cooking}_excerpt.mp4: excerpts of the demo's clips
 
-The reference (/root/reference, showlab/videollm-online @ e2c78ec) has no numeric tests, so these
+Each reads a checkout of the reference (VLO_REFERENCE), the first two with transformers, the third with OpenCV;
+the tests need only the fixtures.
+The reference (showlab/videollm-online @ e2c78ec) has no numeric tests, so these
 fixtures are the pin for oracle/vlo_oracle.py: same seeded weights (videollm_online_b200.weights),
 same inputs, outputs of `LiveLlamaForCausalLM` / `_siglip_vision_encode` / `fast_greedy_generate` /
 `LiveInfer` methods executed unmodified under transformers 5.5.0.  Import recipe from SURVEY.md §8(c):
 import transformers.Trainer first, insert a stub `peft`, shim torchvision.io.read_video.
-The fixtures travel to the GPU box; /root/reference does not.
 """
+import hashlib
 import importlib.machinery
+import json
 import os
 import pathlib
 import sys
@@ -308,5 +313,73 @@ def main():
         print(k, tuple(v.shape) if isinstance(v, torch.Tensor) else v)
 
 
+def digest(t: torch.Tensor) -> str:
+    """SHA-256 of a tensor's dtype, shape and raw bytes: equal digests <=> bit-identical tensors."""
+    h = hashlib.sha256(f"{t.dtype} {tuple(t.shape)}".encode())
+    h.update(t.detach().contiguous().reshape(-1).view(torch.uint8).numpy().tobytes())
+    return h.hexdigest()
+
+
+def bf16_gemm_fingerprint(cfg) -> str:
+    """Digest of plain bf16 CPU GEMMs at the tiny decoder's projection shapes.  torch picks its bf16 GEMM kernel by
+    ISA (AMX / avx512_bf16 / AVX-512 accumulate in different orders), so two hosts with the same fingerprint compute
+    the same bf16 forward bit for bit, and hosts with different ones may differ by an ulp."""
+    g = torch.Generator().manual_seed(0)
+    h = hashlib.sha256()
+    q = cfg.num_attention_heads * cfg.head_dim
+    for m in (1, 11, 17):
+        for k, n in ((cfg.hidden_size, q), (cfg.hidden_size, cfg.intermediate_size), (cfg.intermediate_size, cfg.hidden_size),
+                     (cfg.hidden_size, cfg.vocab_size)):
+            x = torch.randn(m, k, generator=g).to(torch.bfloat16)
+            w = torch.randn(n, k, generator=g).to(torch.bfloat16)
+            h.update(torch.nn.functional.linear(x, w).view(torch.uint8).numpy().tobytes())
+    return h.hexdigest()
+
+
+@torch.no_grad()
+def forward_digests():
+    """reference_forward.json: digests of the reference's forward on the inputs of tiny_reference.pt (per-chunk logits
+    of the KV-append forward, last-layer K / V, logits of forward(input_ids, frames)) and the GEMM fingerprint of the
+    host that ran it.  Stored as digests because the claim they carry is bit-identity on such a host."""
+    cfg = tiny_config()
+    llm_state = W.synthetic_llm_state(cfg, seed=0)
+    llm_state["lm_head.weight"] = (llm_state["lm_head.weight"].float() * 8).to(torch.bfloat16)
+    model, _, _ = build_reference_model(cfg, llm_state, W.synthetic_vision_state(cfg, seed=1))
+    fx = torch.load(OUT / "tiny_reference.pt", weights_only=False)
+    rec, cache, off = {"bf16_gemm_fingerprint": bf16_gemm_fingerprint(cfg), "chunk_logits": []}, None, 0
+    for c in fx["step_chunks"].tolist():
+        out = model(inputs_embeds=fx["step_embeds"][None, off:off + c], use_cache=True, past_key_values=cache)
+        cache = out.past_key_values
+        rec["chunk_logits"].append(digest(out.logits[0]))
+        off += c
+    L = cfg.num_hidden_layers - 1
+    rec["kv_kL"], rec["kv_vL"] = digest(cache.layers[L].keys[0]), digest(cache.layers[L].values[0])
+    rec["joint_logits"] = digest(model(input_ids=fx["joint_ids"], frames=fx["frames"][:2], use_cache=False).logits[0])
+    (OUT / "reference_forward.json").write_text(json.dumps(rec, indent=1) + "\n")
+    print(json.dumps(rec, indent=1))
+
+
+def demo_clip_excerpts():
+    """The first second of the two clips the reference's demo plays (demo/assets/cooking.mp4 1440x1080, bicycle.mp4
+    512x384, 30 fps), as the 2 FPS ingest sees it: source frames 0 and 15, each held for 15 frames, 30 fps, MPEG-4
+    part 2 (the encoder OpenCV ships).  cooking is scaled to 480x360 (same 4:3 letterbox) to keep the file small."""
+    import cv2
+    for name, size in (("bicycle", None), ("cooking", (480, 360))):
+        cap = cv2.VideoCapture(os.path.join(REF, "demo", "assets", name + ".mp4"))
+        src = [cap.read()[1] for _ in range(30)]
+        cap.release()
+        if size is not None:
+            src = [cv2.resize(f, size, interpolation=cv2.INTER_AREA) for f in src]
+        h, w = src[0].shape[:2]
+        path = OUT / f"demo_{name}_excerpt.mp4"
+        wr = cv2.VideoWriter(str(path), cv2.CAP_FFMPEG, cv2.VideoWriter_fourcc(*"mp4v"), 30.0, (w, h),
+                             [cv2.VIDEOWRITER_PROP_KEY_INTERVAL, 1000])
+        for i in range(30):
+            wr.write(src[i - i % 15])
+        wr.release()
+        print(path, w, h, path.stat().st_size)
+
+
 if __name__ == "__main__":
-    main()
+    # no argument: tiny_reference.pt; `forward`: reference_forward.json; `clips`: the demo clip excerpts
+    {"forward": forward_digests, "clips": demo_clip_excerpts}.get(sys.argv[1] if len(sys.argv) > 1 else None, main)()

@@ -274,16 +274,14 @@ def test_video_ingest_matches_ffmpeg_once_geometry(tmp_path):
 
 
 def test_video_ingest_of_the_reference_demo_clips():
-    """The clips demo/cli.py:12 plays (demo/assets/cooking.mp4 1440x1080, bicycle.mp4 512x384, 30 fps, ~100 s): streamed
-    through the ingest at the demo's 2 FPS / 384 px.  Build container only (the reference checkout does not travel)."""
+    """The clips demo/cli.py:12 plays (demo/assets/cooking.mp4 1440x1080, bicycle.mp4 512x384, 30 fps), streamed through
+    the ingest at the demo's 2 FPS / 384 px: their first second as stored in tests/golden (make_golden.py clips; cooking
+    scaled to 480x360, the same 4:3 letterbox)."""
     pytest.importorskip("cv2")
-    import os
     from videollm_online_b200.video_ingest import letterbox_geometry, read_video_resampled
-    root = os.path.join(os.environ.get("VLO_REFERENCE", "/root/reference"), "demo", "assets")
-    if not os.path.isfile(os.path.join(root, "cooking.mp4")):
-        pytest.skip("reference demo assets not present")
-    for name, (w, h, n_src) in {"cooking.mp4": (1440, 1080, 3204), "bicycle.mp4": (512, 384, 3000)}.items():
-        v = read_video_resampled(os.path.join(root, name), fps=2, resolution=384)
+    assert letterbox_geometry(1440, 1080, 384) == (384, 288, 0, 48)
+    for name, (w, h, n_src) in {"cooking": (480, 360, 30), "bicycle": (512, 384, 30)}.items():
+        v = read_video_resampled(str(ROOT / "tests" / "golden" / f"demo_{name}_excerpt.mp4"), fps=2, resolution=384)
         n_out = round(n_src / 30.0 * 2)
         assert v.dtype == torch.uint8 and tuple(v.shape) == (n_out, 3, 384, 384), (name, tuple(v.shape))
         sw, sh, x0, y0 = letterbox_geometry(w, h, 384)

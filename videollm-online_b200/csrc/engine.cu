@@ -42,7 +42,8 @@ struct vlo_engine {
   int device = 0;
   // Cluster kernels (the 2-CTA ViT GEMMs) never run concurrently with a decoder step: next to the step's deep PDL chain
   // (several kernels resident early, all SM shared memory taken) a pending CTA pair was observed to stall both streams.
-  // A step enqueued on another stream than the last pair-GEMM ViT pass waits for that pass, and vice versa (events below).
+  // A step enqueued on another stream than the last pair-GEMM ViT pass waits for that pass, and vice versa (events below);
+  // on one stream a pair-GEMM pass starts with a kernel launched without PDL (vlo_vit_encode), and a step starts with copies.
   cudaEvent_t ev_step = nullptr, ev_pair = nullptr;
   cudaStream_t step_stream = nullptr, pair_stream = nullptr;
   bool step_seen = false, pair_seen = false;
@@ -625,12 +626,30 @@ int vlo_vit_encode(vlo_engine* e, const uint8_t* d_frames, int B, void* d_out, f
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
   const int C = c.vit_hidden, M = c.vit_mlp, P = e->n_patches, rows = B * P;
   const size_t ln_smem = static_cast<size_t>(C) * sizeof(float);
+  // Batches of >= 3 frames (encode-ahead groups, multi-stream ticks, offline extraction) are tensor-bound: their trunk
+  // GEMMs run on CTA pairs (tcgen05 cta_group::2, 256 x 256 tiles, gemm2.cuh) with tokens on MMA-M; out_proj / fc2 add
+  // straight into the fp32 residual stream and a plain LayerNorm kernel follows.  VLO_VIT_GEMM2=0: single-CTA path.
+  static int use_gemm2 = -1;
+  if (use_gemm2 < 0) {
+    const char* ev = getenv("VLO_VIT_GEMM2");
+    use_gemm2 = (ev != nullptr && ev[0] == '0') ? 0 : 1;
+  }
+  const bool pair_gemm = use_gemm2 && B >= 3 && C % 128 == 0 && M % 128 == 0;
 
   // K1/K2: normalise + patchify, then patch-embed GEMM with bias + position embedding epilogue
   {
     const long long total = static_cast<long long>(rows) * e->patch_k / 8;
-    VLO_CUDA(launch_pdl(patchify_kernel, dim3(static_cast<unsigned>(std::min<long long>((total + 255) / 256, 4096))), dim3(256), 0, st,
-                        d_frames, e->patches, B, c.image_size, c.patch_size));
+    const dim3 pgrid(static_cast<unsigned>(std::min<long long>((total + 255) / 256, 4096)));
+    if (pair_gemm) {
+      // A pair-GEMM pass must not share the GPU with a decoder step (see vlo_engine::ev_step) on the SAME stream either:
+      // launched with the PDL attribute, this kernel and the early-triggering kernels after it would let the pass's
+      // cluster kernels launch while the tail of a preceding step is still resident, which stalls the GPU.  Without
+      // the attribute the pass starts after everything before it on the stream has finished.
+      patchify_kernel<<<pgrid, 256, 0, st>>>(d_frames, e->patches, B, c.image_size, c.patch_size);
+      VLO_LAUNCH_CHECK();
+    } else {
+      VLO_CUDA(launch_pdl(patchify_kernel, pgrid, dim3(256), 0, st, d_frames, e->patches, B, c.image_size, c.patch_size));
+    }
     count_launch();
     GemmCall g{};
     g.fmt = FMT_F16;
@@ -793,15 +812,6 @@ int vlo_vit_encode(vlo_engine* e, const uint8_t* d_frames, int B, void* d_out, f
   VLO_CUDA(launch_pdl(layernorm_kernel<float>, dim3(rows), dim3(256), ln_smem, st, static_cast<const float*>(e->v_h),
                       e->vit[0].ln1_w, e->vit[0].ln1_b, e->v_xn, static_cast<float*>(nullptr), C, c.vit_ln_eps));
   count_launch();
-  // Batches of >= 3 frames (encode-ahead groups, multi-stream ticks, offline extraction) are tensor-bound: their trunk
-  // GEMMs run on CTA pairs (tcgen05 cta_group::2, 256 x 256 tiles, gemm2.cuh) with tokens on MMA-M; out_proj / fc2 add
-  // straight into the fp32 residual stream and a plain LayerNorm kernel follows.  VLO_VIT_GEMM2=0: single-CTA path.
-  static int use_gemm2 = -1;
-  if (use_gemm2 < 0) {
-    const char* ev = getenv("VLO_VIT_GEMM2");
-    use_gemm2 = (ev != nullptr && ev[0] == '0') ? 0 : 1;
-  }
-  const bool pair_gemm = use_gemm2 && B >= 3 && C % 128 == 0 && M % 128 == 0;
   if (pair_gemm) {
     if (e->ev_pair == nullptr) VLO_CUDA(cudaEventCreateWithFlags(&e->ev_pair, cudaEventDisableTiming));
     if (e->step_seen && e->step_stream != st) VLO_CUDA(cudaStreamWaitEvent(st, e->ev_step, 0));   // behind the last decoder step
